@@ -74,12 +74,19 @@ def parse_args():
     ap.add_argument('--driver', default='own', choices=['own', 'reference'],
                     help="'reference': the unmodified tenpy TwoSiteDMRGEngine (tenpy_b200.dropin) drives the sweep on the device "
                          "engine instead of tenpy_b200.algorithms.dmrg (short line; the default run reports it as `reference_driver`)")
-    ap.add_argument('--ref-budget-s', type=float, default=240., help='--impl reference: wall-clock budget of the measured steps')
     ap.add_argument('--scan', default='auto', choices=['auto', 'on', 'off'],
                     help='BASELINE.json configs[4]: chi in {256,512,1024,2048} x two fields, sharded over the ranks by LPT '
                          '(tenpy_b200.scan); auto = on for N > 1')
     ap.add_argument('--scan-chis', default='256,512,1024,2048')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed sweep computed (energies, truncation errors, Schmidt values, a seeded '
+                         'sample of the MPS tensors) to DIR/<name>.npy, float64, rank 0 only; default workload only')
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'b200' or args.workload != 'tfi' or args.driver != 'own'):
+        ap.error('--dump-outputs applies to the default workload of the b200 arm only')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 def measured_peaks():
@@ -241,8 +248,8 @@ def synthetic_tensors_host(L, chi, d, seed):
 
 
 class ReferenceArm:
-    """The unmodified reference (tenpy from ``baseline/_ref`` -- the offline pip install with the compiled Cython helper --
-    or the read-only checkout) on the host cores: its own TFIChain, MPS, MPOEnvironment and TwoSiteDMRGEngine on its own
+    """The unmodified reference (tenpy from ``oracle/_ref`` -- the install with the compiled Cython helper that ``build()``
+    makes -- or ``$TENPY_REFERENCE``) on the host cores: its own TFIChain, MPS, MPOEnvironment and TwoSiteDMRGEngine on its own
     NumPy / BLAS / LAPACK engine, the same synthetic state and options as the GPU arm.  A full sweep at chi = 1024 takes
     10-20 minutes on the CPU, so one step is a BOUNDED SAMPLE: `n_bonds` bond updates at the chain centre through
     ``engine.sweep()`` with the schedule restricted to these bonds, scaled to the 158 full-chi bonds of a sweep
@@ -252,7 +259,7 @@ class ReferenceArm:
         from tenpy_b200 import dropin
         self.path = dropin.reference_path()
         if self.path is None:
-            raise RuntimeError('no reference install (baseline/_ref) or checkout found')
+            raise RuntimeError('no reference install (oracle/_ref) or $TENPY_REFERENCE found')
         if self.path not in sys.path:
             sys.path.insert(0, self.path)
         import tenpy
@@ -325,7 +332,7 @@ class ReferenceArm:
 
 def reference_components_sample(args, budget_s=40.):
     """`cpu_baseline` of the GPU arm's line: the pieces of ONE centre-bond update timed on the unmodified reference's own
-    engine (tenpy.linalg.np_conserved from baseline/_ref: `npc.tensordot` for the two contractions of `TwoSiteH.matvec`,
+    engine (tenpy.linalg.np_conserved from oracle/_ref: `npc.tensordot` for the two contractions of `TwoSiteH.matvec`,
     `npc.svd` of the two-site wave function of the benchmark state), without building the 2 x 49 environments a real sweep
     needs (the `--impl reference` arm does that): bond = N_lanczos matvecs + SVD + environment update (3/4 matvec,
     SURVEY.md section 8a9).  Returns None when no reference is installed."""
@@ -405,21 +412,13 @@ def run_reference(args):
         cores, extra = blas_threads(), {'fallback_reason': why, 'matvec_s': vals[0]['matvec_s']}
         sample = '1 centre-bond update per step with the dense numpy port oracle/dmrg_dense.py (reference not installed here)'
     else:
-        t_start = time.perf_counter()
         arm.step(1)                               # builds the 2 x 49 environments up to the centre (not timed)
         threads = arm.choose_threads()
-        # one bond update of this workload takes 5-50 s on the host (LAPACK on a numerically low-rank 2048 x 2048 theta), so
-        # the K + W steps the driver asks for are measured within a time budget; later steps reuse the mean so far
-        per, skipped = [], 0
-        for it in range(args.warmup + args.steps):
-            if per and time.perf_counter() - t_start > args.ref_budget_s:
-                skipped += 1
-                continue
-            dt = arm.step(1)
-            if it >= args.warmup or (it == args.warmup + args.steps - 1 and not per):
-                per.append(dt)
-            elif time.perf_counter() - t_start > args.ref_budget_s and not per:
-                per.append(dt)                    # the budget is gone after the warm-up steps: their last one counts
+        # one bond update of this workload takes 5-50 s on the host (LAPACK on a numerically low-rank 2048 x 2048 theta):
+        # W warm-up steps, then exactly K timed ones
+        for _ in range(args.warmup):
+            arm.step(1)
+        per = [arm.step(1) for _ in range(args.steps)]
         per_bond = float(np.mean(per))
         full = n_full_bonds(args.L, args.chi, 2)
         cores = threads
@@ -428,8 +427,7 @@ def run_reference(args):
                  'thread_sweep': {str(k): v for k, v in sw.items()}, 'matvec_s': sw[threads]['matvec_s'],
                  'svd_s': sw[threads]['svd_s'],
                  'matvec_gflops': 4. * 3 * 8 * float(args.chi)**3 / sw[threads]['matvec_s'] / 1e9,
-                 'per_bond_s_each_step': per, 'steps_measured': len(per), 'steps_not_run_time_budget': skipped,
-                 'time_budget_s': args.ref_budget_s}
+                 'per_bond_s_each_step': per, 'steps_measured': len(per)}
         sample = ('1 bond update at the chain centre per step through the unmodified tenpy TwoSiteDMRGEngine.sweep() '
                   '(schedule restricted to that bond; %d Lanczos matvecs LHeff.theta.RHeff + LAPACK SVD + environment '
                   'update, %d BLAS threads = best of the thread sweep), x %d full-chi bonds of a sweep'
@@ -514,6 +512,42 @@ def psi_from_host(psi, host_bufs):
     return nbytes
 
 
+DUMP_MAX_BYTES = (64 << 20) - 4096     # all files of --dump-outputs together, .npy headers included
+
+
+def _seeded_sample(a, k, rng):
+    """all of `a` if it has at most `k` entries, else `k` of them chosen by `rng` (in index order)"""
+    return a if a.size <= k else a[np.sort(rng.choice(a.size, k, replace=False))]
+
+
+def dump_outputs(out_dir, eng, psi, L):
+    """What a caller of the timed sweep receives, as float64 .npy files of at most DUMP_MAX_BYTES together: the energy and
+    truncation error of each bond update of the last sweep, the Schmidt values of every bond (zero-padded to the largest
+    bond dimension; a seeded sample of that array if it would take more than a quarter of the budget) and a seeded sample
+    of every MPS tensor in right-canonical form, (vL, p, vR) order (all entries of a small tensor; the same entries for
+    the same shapes)."""
+    os.makedirs(out_dir, exist_ok=True)
+    nb = 2 * (L - 2)
+    energy = np.asarray([float(e) for e in eng.update_stats['E_total'][-nb:]], np.float64)
+    err = np.asarray([float(getattr(e, 'eps', e)) for e in eng.update_stats['err'][-nb:]], np.float64)
+    budget = DUMP_MAX_BYTES // 8 - energy.size - err.size           # float64 entries left for S and the B sample
+    Ss = [np.asarray(s.detach().cpu() if hasattr(s, 'detach') else s, np.float64).ravel() for s in psi._S]
+    S = np.zeros((len(Ss), max(len(s) for s in Ss)), np.float64)
+    for i, s in enumerate(Ss):
+        S[i, :len(s)] = s
+    rng = np.random.default_rng(0)
+    if S.size > budget // 4:
+        S = _seeded_sample(S.ravel(), budget // 4, rng)
+    per_site = (budget - S.size) // L
+    samples = []
+    for i in range(L):
+        B = psi.get_B(i, 'B')
+        dense = B.to_ndarray().transpose([B.get_leg_labels().index(l) for l in ('vL', 'p', 'vR')]).ravel()
+        samples.append(_seeded_sample(dense, per_site, rng))
+    for name, a in (('energy', energy), ('trunc_err', err), ('schmidt_values', S), ('B_sample', np.concatenate(samples))):
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -573,6 +607,8 @@ def run_b200(args):
     launches = lib.kernel_launch_count()
     ms = ev0.elapsed_time(ev1) / args.steps
     clocks = sampler.summary() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, psi, L)
     E_final = eng.update_stats['E_total'][-1]
     S_mid = eng._entropy_approx[L // 2]
     N_lan = float(np.mean(eng.update_stats['N_lanczos'][-2 * (L - 2):]))
@@ -1045,7 +1081,7 @@ def run_b200_reference_driver(args):
     lib = backend.use_library(DeviceLib())
     path = dropin.install()
     if path is None:
-        print(json.dumps({'driver': 'reference', 'unavailable': 'no reference install (baseline/_ref)'}))
+        print(json.dumps({'driver': 'reference', 'unavailable': 'no reference install (oracle/_ref)'}))
         return
     import tenpy
     from tenpy.models.tf_ising import TFIChain

@@ -37,9 +37,9 @@ _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def reference_path():
-    """where the unmodified reference lives: ``$TENPY_REFERENCE``, the offline install ``baseline/_ref`` next to the
-    package (travels to the GPU box), or the read-only checkout of the build container"""
-    cands = [os.environ.get('TENPY_REFERENCE'), os.path.join(_ROOT, 'baseline', '_ref'), '/root/reference']
+    """where the unmodified reference lives: ``$TENPY_REFERENCE``, or the install ``oracle/_ref`` that ``build()`` makes
+    from a reference checkout (oracle/reference_install.py)"""
+    cands = [os.environ.get('TENPY_REFERENCE'), os.path.join(_ROOT, 'oracle', '_ref')]
     for c in cands:
         if c and os.path.isdir(os.path.join(c, 'tenpy')):
             return c

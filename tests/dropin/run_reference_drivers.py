@@ -32,7 +32,7 @@ def setup(mode):
         from tenpy_b200._lib import DeviceLib
         backend.use_library(DeviceLib())
     path = dropin.install()
-    assert path is not None, 'reference not found (baseline/_ref)'
+    assert path is not None, 'reference not found (oracle/_ref)'
     import tenpy
     import tenpy.linalg.np_conserved as npc
     assert npc.__name__ == 'tenpy_b200.linalg.np_conserved', npc.__name__

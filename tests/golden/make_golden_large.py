@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Goldens for BASELINE.json configs[2] / [3] at the largest size the reference finishes in the build container in a few
 minutes: two-site DMRG of SpinChain (XXZ, U(1) Sz) and FermiHubbardChain (U(1) x U(1): N, Sz) with the density-matrix
-mixer and a bond-dimension ramp, run by the UNMODIFIED reference (compiled Cython helper, baseline/_ref).  Writes
+mixer and a bond-dimension ramp, run by the UNMODIFIED reference (compiled Cython helper, oracle/_ref).  Writes
 tests/golden/dmrg_large.json: energy, entanglement entropies, bond dimensions, centre Schmidt values, sweep times.
 
     python tests/golden/make_golden_large.py [xxz|hubbard ...]

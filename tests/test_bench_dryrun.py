@@ -6,13 +6,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_bench_contract_keys_dry_run():
+def test_bench_contract_keys_dry_run(tmp_path):
     out = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'dev_bench_dryrun.py'), '--L', '12', '--chi', '16',
-                          '--steps', '1', '--warmup', '1', '--cpu-bonds', '1'], capture_output=True, text=True,
-                         timeout=600, cwd=ROOT)
+                          '--steps', '1', '--warmup', '1', '--cpu-bonds', '1', '--dump-outputs', str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith('{')]
     assert len(lines) == 1, out.stdout[-2000:]
@@ -30,6 +32,27 @@ def test_bench_contract_keys_dry_run():
     assert 'error' not in d['matvec_orders'] and 'error' not in d['roofline_svd']['workload_theta']
     assert all('error' not in p for p in d['blocksparse_matvec'])
     assert 'E_rel_err' in d['parity'] and 'E_exact_free_fermion' in d['parity']
+    # --dump-outputs: the last timed sweep's results (L = 12: 20 bond updates, 13 bonds, every tensor entry kept)
+    dump = {n: np.load(os.path.join(str(tmp_path), n + '.npy')) for n in ('energy', 'trunc_err', 'schmidt_values', 'B_sample')}
+    assert all(a.dtype == np.float64 for a in dump.values())
+    assert dump['energy'].shape == dump['trunc_err'].shape == (20,) and dump['schmidt_values'].shape == (13, 16)
+    assert abs(dump['energy'][-1] - d['result']['E'][0]) < 1e-12 * abs(dump['energy'][-1])
+    dims = [min(2**i, 2**(12 - i), 16) for i in range(13)]
+    assert dump['B_sample'].size == sum(dims[i] * 2 * dims[i + 1] for i in range(12))
+    # the dumped right-canonical tensors are the final state: their product is normalised and has the last bond energy
+    # (TFIChain J = g = 1: H = -sum X_i X_i+1 - sum Z_i)
+    psi, at = np.ones(1), 0
+    for i in range(12):
+        n = dims[i] * 2 * dims[i + 1]
+        psi = np.tensordot(psi.reshape(-1, dims[i]), dump['B_sample'][at:at + n].reshape(dims[i], 2, dims[i + 1]), axes=[1, 0])
+        at += n
+    psi = psi.reshape([2] * 12)
+    X, Z = np.array([[0., 1.], [1., 0.]]), np.diag([1., -1.])
+
+    def op(o, i, v):
+        return np.moveaxis(np.tensordot(o, v, axes=[1, i]), 0, i)
+    E = -sum(np.vdot(psi, op(X, i, op(X, i + 1, psi))) for i in range(11)) - sum(np.vdot(psi, op(Z, i, psi)) for i in range(12))
+    assert abs(np.vdot(psi, psi) - 1.) < 1e-12 and abs(E - dump['energy'][-1]) < 1e-10 * abs(E), (np.vdot(psi, psi), E)
 
 
 def test_bench_reference_arm():
@@ -37,7 +60,7 @@ def test_bench_reference_arm():
                           '--steps', '1', '--warmup', '0'], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     d = json.loads(out.stdout.strip().splitlines()[-1])
-    # the unmodified reference (baseline/_ref or the checkout) when it is there, the dense numpy port otherwise
+    # the unmodified reference (oracle/_ref or $TENPY_REFERENCE) when it is there, the dense numpy port otherwise
     assert d['impl'] == 'reference' and d['cpu_baseline']['kind'] in ('reference', 'port') and d['e2e']['h2d_bytes_per_step'] == 0
     assert d['value'] > 0 and d['config']['chi'] == 32 and d['extrapolated'] is True
     if d['cpu_baseline']['kind'] == 'reference':

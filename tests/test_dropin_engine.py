@@ -3,8 +3,8 @@
 
 Each case runs in its own process (the engine has to be seeded before the first ``import tenpy``;
 tests/dropin/run_reference_drivers.py) and is compared with the numbers the plain reference gives on its NumPy engine
-(tests/golden/dropin.json, written by ``run_reference_drivers.py golden``).  The reference is taken from ``baseline/_ref``
-(offline install, travels to the GPU box) or ``/root/reference``; without either the tests skip."""
+(tests/golden/dropin.json, written by ``run_reference_drivers.py golden``).  The reference is taken from ``$TENPY_REFERENCE``
+or the install ``oracle/_ref`` that ``build()`` makes from a reference checkout; without either the tests skip."""
 import json
 import os
 import subprocess
@@ -45,7 +45,7 @@ def _check(case, got):
 def test_reference_drivers_on_engine_host_logic(case):
     """numpy test double of the device library: the engine's host logic under the reference's drivers"""
     if not _reference_available():
-        pytest.skip('no reference checkout / install (baseline/_ref)')
+        pytest.skip('no reference install (oracle/_ref, built from a reference checkout)')
     _check(case, _run('fake', case))
 
 
@@ -55,5 +55,5 @@ def test_reference_drivers_on_engine_gpu(case, gpu_lib):
     """the same on the B200: every Array of the reference's DMRG / TEBD run lives in HBM, every contraction / SVD / eigh /
     block move is a kernel of libb200npc.so"""
     if not _reference_available():
-        pytest.skip('no reference install on this box (baseline/_ref)')
+        pytest.skip('no reference install (oracle/_ref, built from a reference checkout)')
     _check(case, _run('cuda', case))

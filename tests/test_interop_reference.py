@@ -1,7 +1,7 @@
 """Checkpoint exchange with the UNMODIFIED reference (SURVEY.md section 8f rank 4): a DMRG state computed by this package
 is converted with `tenpy_b200.tools.interop`, pickled, loaded by stock TeNPy (which measures the same energy and
-continues the run), and a reference state comes back.  Needs the reference (the checkout of the build container or the
-offline install baseline/_ref that travels to the GPU box).  Twice: on the numpy test double (host logic) and, ``-m gpu``, with
+continues the run), and a reference state comes back.  Needs the reference (``$TENPY_REFERENCE`` or the
+install oracle/_ref that ``build()`` makes from a reference checkout).  Twice: on the numpy test double (host logic) and, ``-m gpu``, with
 the state computed and re-imported on the B200."""
 import os
 import subprocess
@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from tenpy_b200 import dropin  # noqa: E402
 
-REF = os.environ.get('TENPY_REFERENCE') or dropin.reference_path() or '/root/reference'
+REF = dropin.reference_path() or ''
 
 SCRIPT = r'''
 import sys, pickle, warnings, io
@@ -85,6 +85,6 @@ def test_checkpoint_roundtrip_with_reference(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'tenpy')), reason='reference not available (baseline/_ref)')
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'tenpy')), reason='reference not available (oracle/_ref)')
 def test_checkpoint_roundtrip_with_reference_gpu(tmp_path, gpu_lib):
     _roundtrip(tmp_path, False)

@@ -11,7 +11,7 @@ from test_tebd import _run, _reference_available
 
 def _check(mode):
     if not _reference_available():
-        pytest.skip('no reference checkout / install (baseline/_ref)')
+        pytest.skip('no reference install (oracle/_ref, built from a reference checkout)')
     res = _run(mode, 'qr_trunc_golden')
     assert res['cases'] == 8 and res['max_iso_err'] < 1e-11
 

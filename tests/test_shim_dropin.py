@@ -1,7 +1,7 @@
 """CPU test of the drop-in boundary B2 (SURVEY.md section 8b): the UNMODIFIED reference (tenpy/tenpy) runs its own
 two-site DMRG with `tenpy.linalg._npc_helper` replaced by `tenpy_b200.shim._npc_helper` through the
 reference's plugin switch `tools.optimization.use_cython` (doc-string check included).  Needs the reference
-checkout (/root/reference, build container only) -> skipped on the GPU box; device calls go to the numpy test
+(`tenpy_b200.dropin.reference_path`), skipped without it; device calls go to the numpy test
 double here (host logic of the shim), the kernels themselves are covered by the -m gpu tests."""
 import os
 import subprocess
@@ -10,7 +10,10 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get('TENPY_REFERENCE', '/root/reference')
+sys.path.insert(0, ROOT)
+from tenpy_b200 import dropin  # noqa: E402
+
+REF = dropin.reference_path() or ''
 
 SCRIPT = r'''
 import sys, warnings
@@ -48,7 +51,7 @@ print('E=%.12f' % res['E'])
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'tenpy')), reason='reference checkout not available')
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'tenpy')), reason='reference not available')
 def test_reference_dmrg_runs_on_the_shim(tmp_path):
     script = tmp_path / 'dropin.py'
     script.write_text(SCRIPT.format(root=ROOT, ref=REF))

@@ -43,7 +43,7 @@ def _compare(got, g, tags, eps_tol, tol=1e-9):
 
 def _check_tebd(mode):
     if not _reference_available():
-        pytest.skip('no reference checkout / install (baseline/_ref)')
+        pytest.skip('no reference install (oracle/_ref, built from a reference checkout)')
     got, g = _run(mode, 'tebd_golden'), h.load('tebd.npz')
     for name in ('tfi', 'tfip', 'xxz', 'hub'):
         assert np.max(np.abs(np.array(got[name + '_Hbond_mid']) - g[name + '_Hbond_mid'])) < 1e-14
@@ -54,7 +54,7 @@ def _check_tebd(mode):
 
 def _check_tebd_qr(mode):
     if not _reference_available():
-        pytest.skip('no reference checkout / install (baseline/_ref)')
+        pytest.skip('no reference install (oracle/_ref, built from a reference checkout)')
     got, g = _run(mode, 'tebd_qr_golden'), h.load('tebd_qr.npz')
     _compare(got, g, [n + t for n in ('tfi', 'xxz') for t in ('_imag', '_o2')], lambda e: 1e-13)
 

@@ -1,52 +1,33 @@
 """`tenpy_b200.linalg.truncation.truncate` (own formulation: conditions on the number of kept values) against the
 reference's `truncate` (truncation.py:146) on randomised spectra and option combinations: same number of kept values, same
-norm, same truncation error.  Needs the reference (baseline/_ref or the checkout); skips otherwise."""
-import os
-import sys
+norm, same truncation error.  Inputs and the reference's outputs are stored in tests/golden/truncate.npz (written by
+tests/golden/make_golden_truncate.py)."""
 import warnings
 
 import numpy as np
-import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+import helpers as h
+
+OPTION_KEYS = ('chi_max', 'chi_min', 'degeneracy_tol', 'svd_min', 'trunc_cut')
+INT_OPTIONS = ('chi_max', 'chi_min')
+
+
+def _trials(g):
+    for i in range(len(g['n'])):
+        opts = {}
+        for key in OPTION_KEYS:
+            if g['has_' + key][i]:
+                v = g['opt_' + key][i]
+                opts[key] = None if np.isnan(v) else (int(v) if key in INT_OPTIONS else float(v))
+        yield g['S_pad'][i, :g['n'][i]], opts
 
 
 def test_truncate_matches_reference_randomised():
-    sys.path.insert(0, ROOT)
-    from tenpy_b200 import dropin
     from tenpy_b200.linalg.truncation import truncate as mine
-    path = dropin.reference_path()
-    if path is None or dropin.installed():
-        pytest.skip('plain reference not importable in this process')
-    sys.path.insert(0, path)
-    from tenpy.linalg.truncation import truncate as ref
-    from tenpy.tools.params import Config
-    rng = np.random.default_rng(0)
+    g = h.load('truncate.npz')
+    assert len(g['kept']) == 1500
     with warnings.catch_warnings():
         warnings.simplefilter('ignore')
-        for trial in range(1500):
-            n = int(rng.integers(1, 40))
-            kind = rng.integers(0, 4)
-            if kind == 0:
-                S = rng.random(n)
-            elif kind == 1:
-                S = np.exp(-rng.random(n) * 40)
-            elif kind == 2:
-                S = np.repeat(rng.random(max(1, n // 3)), 3)[:n]
-            else:
-                S = np.concatenate([rng.random(n // 2 + 1), np.zeros(n // 2)])
-            S = S / np.linalg.norm(S)
-            opts = {}
-            if rng.random() < .8:
-                opts['chi_max'] = int(rng.integers(1, 45)) if rng.random() < .9 else None
-            if rng.random() < .3:
-                opts['chi_min'] = int(rng.integers(1, 45))
-            if rng.random() < .3:
-                opts['degeneracy_tol'] = float(10 ** rng.uniform(-8, -1))
-            if rng.random() < .7:
-                opts['svd_min'] = float(10 ** rng.uniform(-16, -1)) if rng.random() < .9 else None
-            if rng.random() < .7:
-                opts['trunc_cut'] = float(10 ** rng.uniform(-16, -0.5)) if rng.random() < .9 else None
+        for (S, opts), k2, n2, e2 in zip(_trials(g), g['kept'], g['norm'], g['eps']):
             m1, n1, e1 = mine(S, dict(opts))
-            m2, n2, e2 = ref(S, Config(dict(opts), 'trunc'))
-            assert m1.sum() == m2.sum() and abs(n1 - n2) < 1e-14 and abs(e1.eps - e2.eps) < 1e-14, (opts, S)
+            assert m1.sum() == k2 and abs(n1 - n2) < 1e-14 and abs(e1.eps - e2) < 1e-14, (opts, S)
